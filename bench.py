@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the hot path (BASELINE.json metric: CTR forward+backward samples/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--ids uniform|zipf]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch.  Workloads (BASELINE.json `configs`):
   deepfm_cfg5          configs[4] on ONE GPU (default at N=1): DeepFM, 40 fields, embed_dim 32, batch 65536, 100 M-row
@@ -203,6 +204,26 @@ def timed_steps(dd: Dist, step, steps, n_marks=0):
     ms = dd.max(t0.elapsed_time(t1))
     marks = [statistics.mean(e[j].elapsed_time(e[j + 1]) for e in evs) for j in range(n_marks)] if evs else []
     return ms, marks
+
+
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(path, whole, per_sample):
+    """--dump-outputs: writes `whole`'s tensors in full and, of `per_sample`'s (batch-major) tensors, the same fixed, seeded
+    sample of batch rows (ascending, as many as keep the total within DUMP_BYTES), as float32 `path/<name>.npy`.  The bench
+    inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: t.detach().float().cpu().numpy() for k, t in whole.items()}
+    B = next(iter(per_sample.values())).shape[0]
+    row_bytes = sum(t[0].numel() * 4 for t in per_sample.values())
+    n = min(B, (DUMP_BYTES - sum(a.nbytes for a in arrays.values())) // row_bytes)
+    rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    for k, t in per_sample.items():
+        arrays[k] = t.detach().index_select(0, rows.to(t.device)).float().cpu().numpy()
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def sustained_run(dd: Dist, step, ms_per_step, units_per_step, seconds=2.0):
@@ -528,11 +549,11 @@ def run_deepfm(args, cfg, dd: Dist):
             ops.embed_fm2_bwd(tile, d_tile, d_fm2, row_grads=row_grads)
             if ev:
                 ev[2].record()
-        return tables, rows, id_sets, ids_desc, step
+        return tables, rows, id_sets, ids_desc, step, row_grads
 
     if not sharded_mode:
         # ------------------------------------------------------------------ one GPU (or N replicas, no exchange step)
-        tables, rows, id_sets, ids_desc, step = replica_setup()
+        tables, rows, id_sets, ids_desc, step, row_grads = replica_setup()
         for i in range(args.warmup):
             step(i)
         dd.barrier()
@@ -541,6 +562,9 @@ def run_deepfm(args, cfg, dd: Dist):
         ms_total, (fwd_ms, bwd_ms) = timed_steps(dd, step, args.steps, n_marks=2)
         clocks = sampler.stop()
         launches = _lib.kernel_launches() - launches0
+        if args.dump_outputs and rank == 0:
+            # the buffers still hold the last timed step: later measurements reuse them
+            dump_outputs(args.dump_outputs, whole={"fm2": fm2}, per_sample={"tile": tile, "row_grads": row_grads})
         value = world * B * args.steps / (ms_total * 1e-3)
         sustained = sustained_run(dd, step, ms_total / args.steps, B)
 
@@ -764,7 +788,7 @@ def run_deepfm(args, cfg, dd: Dist):
     # the zero-traffic split of the same batch (replicated 12.8 GB table) for comparison -- NOT the headline at N > 1
     rep = None
     if not args.no_extra:
-        _t, _rows, _ids, _desc, rstep = replica_setup()
+        _t, _rows, _ids, _desc, rstep, _rg = replica_setup()
         for i in range(3):
             rstep(i)
         rms, _ = timed_steps(dd, rstep, min(args.steps, 50))
@@ -910,12 +934,19 @@ def main():
                     help="sharded workloads: 1 = also time the e2e step as a CUDA-graph replay and report the faster form")
     ap.add_argument("--ids", default="uniform", choices=["uniform", "zipf"],
                     help="id distribution of the synthetic batches (default: uniform = every row an HBM miss)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, at most 60 MB): fm2 in "
+                         "full, tile and row_grads for a fixed, seeded sample of batch rows (replicated DeepFM workloads, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.workload is None:
         # BASELINE config 5 names the row-sharded split: it is the headline whenever there is more than one GPU
         args.workload = "deepfm_cfg5_sharded" if (world > 1 and args.impl == "ours") else "deepfm_cfg5"
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in DEEPFM or DEEPFM[args.workload].get("sharded")):
+        ap.error("--dump-outputs covers the replicated DeepFM workloads of --impl ours only")
     if args.impl == "reference":
         if args.workload in LAYER_WORKLOADS:
             run_reference_arm_layers(args)

@@ -1,10 +1,10 @@
 """Generate tests/golden/*.npz by EXECUTING THE REFERENCE'S OWN LAYER FILES (TEST INFRASTRUCTURE).
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of tangxyw/RecAlgorithm (the reference):
 
-    python oracle/make_golden.py
+    python oracle/make_golden.py REFERENCE_CHECKOUT [OUT_DIR]       # OUT_DIR defaults to tests/golden
 
-The five interaction-layer files are imported verbatim from /root/reference/algorithm with
+The five interaction-layer files are imported verbatim from REFERENCE_CHECKOUT/algorithm with
 ``oracle/tf1_shim`` standing in for TensorFlow 1.14 (see that package's docstring for what
 this does and does not pin).  Each fixture stores the seeded inputs, the injected weights
 (under the TF variable names the reference created), and the reference outputs computed in
@@ -12,11 +12,15 @@ float32 (like the reference) and float64 (anchor).  FM2 and the lookup have no i
 reference function (inline code / TF-internal); their fixtures come from
 ``oracle/layers_np.py`` and are marked ``source='restated'``.
 
-The GPU box has no /root/reference: tests read only the committed .npz files.
+Beside the fixtures it writes ``reference_digests.json``: the SHA-256 of every array of the run.  The tests need no
+reference checkout: they compare the committed fixtures with that record, array by array, and regenerate the restated
+fixtures (``gen_restated``, which runs no reference code) bit for bit.
 """
 from __future__ import annotations
 
+import hashlib
 import importlib.util
+import json
 import os
 import sys
 
@@ -24,8 +28,9 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = "/root/reference/algorithm"
+REF = None                      # REFERENCE_CHECKOUT/algorithm, set by load_reference()
 OUT = os.path.join(ROOT, "tests", "golden")
+DIGESTS = "reference_digests.json"
 
 sys.path.insert(0, os.path.join(HERE, "tf1_shim"))
 sys.path.insert(0, ROOT)
@@ -41,11 +46,26 @@ def _load(relpath, name):
     return mod
 
 
-ref_cross = _load("DCN/cross_layer.py", "ref_cross_layer")
-ref_cin = _load("xDeepFM/cin_layer.py", "ref_cin_layer")
-ref_din = _load("DIN/din_attention.py", "ref_din_attention")
-ref_senet = _load("FiBiNET/senet.py", "ref_senet")
-ref_bilinear = _load("FiBiNET/bilinear_interaction_layer.py", "ref_bilinear")
+def load_reference(checkout):
+    """Import the reference's five interaction-layer files from `checkout` (a tangxyw/RecAlgorithm tree)."""
+    global REF, ref_cross, ref_cin, ref_din, ref_senet, ref_bilinear
+    REF = os.path.join(os.path.abspath(checkout), "algorithm")
+    ref_cross = _load("DCN/cross_layer.py", "ref_cross_layer")
+    ref_cin = _load("xDeepFM/cin_layer.py", "ref_cin_layer")
+    ref_din = _load("DIN/din_attention.py", "ref_din_attention")
+    ref_senet = _load("FiBiNET/senet.py", "ref_senet")
+    ref_bilinear = _load("FiBiNET/bilinear_interaction_layer.py", "ref_bilinear")
+
+
+def fixture_digests(directory):
+    """{fixture file: {array name: sha256 of dtype, shape and bytes}} of every .npz in `directory`."""
+    out = {}
+    for f in sorted(os.listdir(directory)):
+        if f.endswith(".npz"):
+            with np.load(os.path.join(directory, f), allow_pickle=False) as z:
+                out[f] = {k: hashlib.sha256(f"{z[k].dtype.str}{z[k].shape}".encode() + z[k].tobytes()).hexdigest()
+                          for k in sorted(z.files)}
+    return out
 
 
 def trunc_normal(rng, shape, std):
@@ -235,7 +255,7 @@ def gen_restated():
          source="restated:TF1.14 feature_column semantics (SURVEY A.4-A.6) -- parity unpinned")
 
 
-# ---- inline blocks of model_fns: the cited source lines are read from /root/reference at generation time and exec()'d ----
+# ---- inline blocks of model_fns: the cited source lines are read from the reference checkout at generation time and exec()'d ----
 
 class _FakeFC:
     """Stand-in for `tf.feature_column` inside the inline blocks: `fc.input_layer(features, [col])` returns the (B, K)
@@ -364,6 +384,11 @@ def gen_ffm():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) not in (2, 3):
+        raise SystemExit(__doc__)
+    load_reference(sys.argv[1])
+    if len(sys.argv) == 3:
+        OUT = sys.argv[2]
     gen_cross()
     gen_cin()
     gen_din()
@@ -372,3 +397,6 @@ if __name__ == "__main__":
     gen_inline()
     gen_bst()
     gen_ffm()
+    with open(os.path.join(OUT, DIGESTS), "w") as fh:
+        json.dump(fixture_digests(OUT), fh, indent=1, sort_keys=True)
+        fh.write("\n")

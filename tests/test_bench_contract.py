@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
@@ -46,6 +48,58 @@ def test_reference_arm_under_torchrun_env_prints_on_rank_0_only():
     (line,) = _reference_line(("--gpus", "2"), env={"RANK": "0", "WORLD_SIZE": "2", "LOCAL_RANK": "0"})
     d = json.loads(line)
     assert d["n_gpus"] == 2 and "single-process" in d["config"]["note"]
+
+
+def test_dump_outputs_writes_float32_whole_and_one_seeded_row_sample(tmp_path):
+    import numpy as np
+    import torch
+    import bench
+    g = torch.Generator().manual_seed(0)
+    B, F, D = 8192, 40, 32                                             # 2 x 42 MB of tile / row_grads: must be sampled
+    fm2, tile = torch.randn((B, 1), generator=g), torch.randn((B, F, D), generator=g)
+    tile[:, 0, 0] = torch.arange(B)                                    # each row says which it is
+    grads = tile * 2
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), whole={"fm2": fm2}, per_sample={"tile": tile, "row_grads": grads})
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["fm2.npy", "row_grads.npy", "tile.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 * 10 ** 6
+    a = {f: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert a[f].dtype == np.float32 and np.array_equal(a[f], np.load(tmp_path / "b" / f))
+    assert np.array_equal(a["fm2.npy"], fm2.numpy())
+    n = a["tile.npy"].shape[0]
+    assert 0 < n < B and a["tile.npy"].shape == a["row_grads.npy"].shape == (n, F, D)
+    rows = a["tile.npy"][:, 0, 0].astype(np.int64)
+    assert (np.diff(rows) > 0).all() and np.array_equal(a["tile.npy"], tile.numpy()[rows])
+    assert np.array_equal(a["row_grads.npy"], grads.numpy()[rows])   # the same rows of every sampled output
+
+
+def test_bench_rejects_zero_steps_and_dumps_it_cannot_make():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"], ["--workload", "dcn_cfg2", "--dump-outputs", "x"],
+                  ["--workload", "deepfm_small_sharded", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=300)
+        assert out.returncode == 2 and "error:" in out.stderr and not out.stdout, extra
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_the_last_timed_step_and_repeat(tmp_path):
+    """Same arguments -> the same dumped outputs; one more timed step -> the last step ran on the next id batch."""
+    import numpy as np
+
+    def run(steps, d):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "deepfm_small", "--steps", str(steps),
+                              "--warmup", "3", "--no-extra", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / d)],
+                             capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        (line,) = [l for l in out.stdout.splitlines() if l.startswith("{")]
+        assert json.loads(line)["steps"] == steps
+        return {f: np.load(tmp_path / d / f) for f in ("fm2.npy", "tile.npy", "row_grads.npy")}
+
+    a, b, c = run(5, "a"), run(5, "b"), run(6, "c")
+    for f in a:
+        assert a[f].dtype == np.float32 and np.isfinite(a[f]).all() and np.array_equal(a[f], b[f]), f
+    assert a["fm2.npy"].shape == (8192, 1) and not np.array_equal(a["fm2.npy"], c["fm2.npy"])
 
 
 def test_algorithmic_bytes_match_survey_8d():

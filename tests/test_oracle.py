@@ -370,24 +370,27 @@ def test_adam_restatement_agrees_with_torch_adam(lazy):
         p_prev = var.copy()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/algorithm"), reason="the reference checkout only exists in the builder container")
 def test_fixtures_regenerate_bit_identically_from_the_reference(tmp_path):
-    """oracle/make_golden.py imports / exec()s the reference's own files over the TF1 shim: run it again (in a subprocess, into a
-    scratch directory) and compare every .npz with the committed fixture, array by array, bit for bit."""
+    """oracle/make_golden.py imports / exec()s the reference's own files over the TF1 shim and records the SHA-256 of every array
+    it made in golden/reference_digests.json.  Every committed fixture must match that record, array by array, bit for bit; the
+    fixtures that run no reference code (gen_restated) are made again here, in a subprocess (the shim goes on sys.path), and must
+    match too."""
+    import json
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = ("import sys, runpy; sys.argv=['make_golden']; import importlib.util as u;"
+    code = ("import sys, json; import importlib.util as u;"
             f"s=u.spec_from_file_location('mg', r'{root}/oracle/make_golden.py'); m=u.module_from_spec(s); s.loader.exec_module(m);"
-            f"m.OUT=r'{tmp_path}';"
-            "[getattr(m, f)() for f in ('gen_cross','gen_cin','gen_din','gen_fibinet','gen_restated','gen_inline','gen_bst','gen_ffm')]")
+            f"m.OUT=r'{tmp_path}'; m.gen_restated();"
+            f"print(json.dumps({{'committed': m.fixture_digests(r'{G}'), 'made': m.fixture_digests(r'{tmp_path}')}}))")
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=900, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
-    made = sorted(glob.glob(os.path.join(str(tmp_path), "*.npz")))
-    committed = sorted(glob.glob(os.path.join(G, "*.npz")))
-    assert [os.path.basename(p) for p in made] == [os.path.basename(p) for p in committed] and len(made) >= 28
-    for a, b in zip(made, committed):
-        x, y = np.load(a, allow_pickle=False), np.load(b, allow_pickle=False)
-        assert sorted(x.files) == sorted(y.files), os.path.basename(a)
-        for k in x.files:
-            assert x[k].dtype == y[k].dtype and x[k].shape == y[k].shape and x[k].tobytes() == y[k].tobytes(), (os.path.basename(a), k)
+    d = json.loads(out.stdout.strip().splitlines()[-1])
+    with open(os.path.join(G, "reference_digests.json")) as fh:
+        recorded = json.load(fh)
+    assert sorted(recorded) == sorted(d["committed"]) and len(recorded) >= 28
+    for f, arrays in recorded.items():
+        assert d["committed"][f] == arrays, f
+    assert sorted(d["made"]) == ["fm2_F40_D32.npz", "fm2_F6_D8.npz", "lookup_edge.npz"]
+    for f, arrays in d["made"].items():
+        assert arrays == recorded[f], f
